@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the abyss-bloom-dbg hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--reads R]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--reads R] [--dump-outputs DIR]
 
 One "step" = one complete pass of the hot path over the synthetic read set:
     pass 1  ntHash of every k-mer of every read + ordered counting-Bloom insert
@@ -252,6 +252,36 @@ def workload_config(args, extra=None):
     return c
 
 
+def dump_outputs(out_dir, asm, filt, read_codes):
+    """--dump-outputs: what a caller of the timed path receives from its last step, as DIR/<name>.npy, so that two builds can
+    be compared output for output: the unitig records in output order (seed read, length, coverage), the unitig bases
+    concatenated in output order (A=0 C=1 G=2 T=3), the per-read result codes (capi.READ_CODES) and the counting filter's
+    counters.  An array longer than its cap is replaced by the entries at sorted positions drawn from
+    np.random.default_rng(SEED).integers(0, length, cap), so the sample depends on the array's length only; the caps keep
+    the directory under 64 MB."""
+    import ctypes
+    import numpy as np
+
+    def sample(a, cap, dtype):
+        if a.size > cap:
+            a = a[np.sort(np.random.default_rng(SEED).integers(0, a.size, cap))]
+        return a.astype(dtype)
+
+    contigs, n, seqs = asm._last
+    recs = np.array([(contigs[i].seed_read, contigs[i].length, contigs[i].coverage) for i in range(n)], dtype=np.float64).reshape(n, 3)
+    base = ctypes.cast(seqs, ctypes.c_void_p).value
+    bases = np.frombuffer(b"".join(ctypes.string_at(base + contigs[i].seq_offset, contigs[i].length) for i in range(n)), dtype=np.uint8)
+    lut = np.full(256, 255, dtype=np.uint8)
+    lut[np.frombuffer(b"ACGT", dtype=np.uint8)] = np.arange(4, dtype=np.uint8)
+    arrays = {"unitig_seed_read": sample(recs[:, 0], 1 << 20, np.float64), "unitig_length": sample(recs[:, 1], 1 << 20, np.float64),
+              "unitig_coverage": sample(recs[:, 2], 1 << 20, np.float64), "unitig_bases": sample(lut[bases], 1 << 22, np.float32),
+              "read_codes": sample(read_codes, 1 << 20, np.float32), "counters": sample(filt.download(), 1 << 22, np.float32)}
+    assert sum(a.nbytes for a in arrays.values()) <= 64_000_000
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -263,7 +293,10 @@ def main():
     ap.add_argument("--window", type=int, default=0, help="ordered-insert window in k-mer slots (0 = library default)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -381,6 +414,8 @@ def main():
     total_kmers = nk  # one job, counted once (strong scaling)
     value = total_kmers / (ms_step * 1e-3)
     digest = asm.last_digests(rs.read_id)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, asm, filt, asm.read_results())
 
     # ---- e2e through host buffers
     e2e = None

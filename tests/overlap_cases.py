@@ -89,6 +89,61 @@ def all_cases():
     return cases
 
 
+def more_fuzz_cases():
+    """further fuzz sets; only the sha256 of the reference's output is stored (overlap_ref_runs.json)"""
+    return [fuzz_case(s) for s in range(1000, 1120)]
+
+
+def cli_cases():
+    """the sets the GPU AdjList command line runs against the reference's output (overlap_ref_runs.json)"""
+    return [fuzz_case(s) for s in range(2000, 2008)] + [tiled_case(9, 1500000, 64, 50, 0), tiled_case(10, 800000, 40, 0, 4)]
+
+
+def alias_runs(tmp_path):
+    """--gv = --dot, --gfa = --gfa1, -m0 = k-1, long options, several input files, contigs on standard input:
+    (name, args, stdin) over two FASTA files written to tmp_path"""
+    c = tiled_case(21, 20000, 31, 20)
+    half = len(c["records"]) // 2
+    a_fa, b_fa = os.path.join(tmp_path, "a.fa"), os.path.join(tmp_path, "b.fa")
+    write_fasta(dict(c, records=c["records"][:half]), a_fa)
+    write_fasta(dict(c, records=c["records"][half:]), b_fa)
+    both = open(a_fa).read() + open(b_fa).read()
+    return [("alias_gv", ["--kmer=31", "--min-overlap=20", "--gv", a_fa, b_fa], None), ("alias_gfa", ["-k31", "-m0", "--gfa", a_fa, b_fa], None),
+            ("alias_stdin_adj", ["-k", "31", "-m", "25", "--SS", "--adj"], both), ("alias_stdin_asqg", ["-k31", "--no-SS", "--asqg", "-"], both)]
+
+
+# config 1 of SURVEY.md 8d (53 333 x 150 bp reads of a 200 kbp genome) through the reference's abyss-bloom-dbg -kK --kc=2 -b64M -H4 -j1:
+# unitig sets with tips, branches and blunt ends from coverage gaps, stored as genome coordinates (unitigs_config1.json.gz)
+UNITIG_SET_READS = (1, 200000, 53333, 150, 0.005)  # ReadSet(seed, genome length, reads, read length, error rate)
+UNITIG_RUNS = [(32, 0, "--adj"), (32, 20, "--dot"), (48, 30, "--gfa1"), (64, 50, "--gfa2"), (96, 50, "--sam"), (40, 25, "--asqg")]
+
+
+def unitig_set_genome():
+    import numpy as np
+    from abyss_b200.synth import ReadSet
+    rs = ReadSet(*UNITIG_SET_READS)
+    return np.frombuffer(b"ACGT", dtype=np.uint8)[rs.genome].tobytes().decode()
+
+
+def unitig_set_fasta(k):
+    """the reference's unitig FASTA at k, rebuilt from unitigs_config1.json.gz: a record is [header, pos, length] (a genome
+    substring; pos < 0: the reverse complement of the one at -pos-1) or [header, sequence] (a unitig that holds read errors)"""
+    import gzip
+    import json
+    sets = json.load(gzip.open(os.path.join(GOLD, "unitigs_config1.json.gz"), "rt"))
+    g = unitig_set_genome()
+    out = []
+    for rec in sets[str(k)]["records"]:
+        if len(rec) == 2:
+            seq = rec[1]
+        elif rec[1] >= 0:
+            seq = g[rec[1]:rec[1] + rec[2]]
+        else:
+            seq = rc(g[-rec[1] - 1:-rec[1] - 1 + rec[2]])
+        out.append(f">{rec[0]}\n{seq}\n")
+    return "".join(out), sets[str(k)]["sha256"]
+
+
 def write_fasta(case, path):
     with open(path, "w") as f:
         for name, comment, seq in case["records"]:
@@ -102,3 +157,11 @@ def command_args(case, fasta_path):
 def normalise(out: bytes, exe: str) -> bytes:
     """the SAM header quotes the command line: make it independent of where the binary lives"""
     return out.replace(exe.encode(), b"AdjList")
+
+
+def ref_run_digest(out: bytes, exe: str, tmp_dir) -> dict:
+    """sha256 and length of an output as overlap_ref_runs.json stores the reference's: independent of where the binary and the
+    input files live"""
+    import hashlib
+    data = normalise(out, exe).replace(str(tmp_dir).encode(), b"TMP")
+    return dict(sha256=hashlib.sha256(data).hexdigest(), bytes=len(data))

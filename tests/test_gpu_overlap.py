@@ -1,6 +1,6 @@
 """GPU: the contig overlap graph (SURVEY.md 8f.3, AdjList/AdjList.cpp) -- the AdjList program over libabyssb200 (CUDA
 hash joins, csrc/abb_overlap.cu) writes the bytes of the unmodified reference AdjList in every output format
-(committed goldens; live against oracle/_ref/AdjList-ref where it travelled), through the C ABI as well, and in the
+(committed goldens of its output), through the C ABI as well, and in the
 pipeline order of bin/abyss-pe: abyss-bloom-dbg -> unitig FASTA -> AdjList."""
 import ctypes as C
 import hashlib
@@ -18,7 +18,6 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(ROOT, "tests", "golden")
 BIN = os.path.join(ROOT, "abyss_b200", "lib")
-REF = os.path.join(ROOT, "oracle", "_ref", "AdjList-ref")
 
 
 def run_case(exe, case, tmp_path):
@@ -44,18 +43,16 @@ def test_cli_goldens(abb, tmp_path):
             assert got == open(full, "rb").read()
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref/AdjList-ref not built")
 def test_cli_live_against_reference(abb, tmp_path):
+    # further sets against the reference's output on them (sha256 in overlap_ref_runs.json)
     exe = os.path.join(BIN, "AdjList")
-    cases = [oc.fuzz_case(s) for s in range(2000, 2008)] + [oc.tiled_case(9, 1500000, 64, 50, 0), oc.tiled_case(10, 800000, 40, 0, 4)]
-    for c in cases:
+    want = json.load(open(os.path.join(GOLD, "overlap_ref_runs.json")))
+    for c in oc.cli_cases():
         fa = str(tmp_path / "in.fa")
         oc.write_fasta(c, fa)
-        a = subprocess.run([REF] + oc.command_args(c, fa), capture_output=True)
-        assert a.returncode == 0, a.stderr.decode()
         b = subprocess.run([exe] + oc.command_args(c, fa), capture_output=True)
         assert b.returncode == 0, b.stderr.decode()
-        assert oc.normalise(a.stdout, REF) == oc.normalise(b.stdout, exe), (c["name"], c["k"], c["m"], c["args"])
+        assert oc.ref_run_digest(b.stdout, exe, tmp_path) == want[c["name"]], (c["name"], c["k"], c["m"], c["args"])
 
 
 def test_c_abi_edges(abb):

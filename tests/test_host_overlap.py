@@ -1,7 +1,7 @@
 """CPU: the overlap-graph join logic (abyss_b200/csrc/abb_overlap.cuh -- the SAME per-item functions the CUDA kernels
 call) and the product's AdjList command line and graph writers (abyss_b200/host/adjlist_main.h), run by the
-single-thread harness tests/host_overlap, against the unmodified reference AdjList: committed goldens
-(tests/golden/make_golden_overlap.py) and, where oracle/_ref/AdjList-ref exists, live on further seeds."""
+single-thread harness tests/host_overlap, against the output of the unmodified reference AdjList (committed goldens,
+tests/golden/make_golden_overlap.py)."""
 import hashlib
 import json
 import os
@@ -13,7 +13,6 @@ import overlap_cases as oc
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(ROOT, "tests", "golden")
-REF = os.path.join(ROOT, "oracle", "_ref", "AdjList-ref")
 
 
 @pytest.fixture(scope="module")
@@ -45,17 +44,15 @@ def test_goldens(harness, tmp_path):
             assert got == open(full, "rb").read()
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref/AdjList-ref not built")
 def test_live_against_reference(harness, tmp_path):
-    for seed in range(1000, 1120):
-        c = oc.fuzz_case(seed)
+    # further fuzz sets against the reference's output on them (sha256 in overlap_ref_runs.json)
+    want = json.load(open(os.path.join(GOLD, "overlap_ref_runs.json")))
+    for c in oc.more_fuzz_cases():
         fa = str(tmp_path / "in.fa")
         oc.write_fasta(c, fa)
-        a = subprocess.run([REF] + oc.command_args(c, fa), capture_output=True)
-        assert a.returncode == 0, a.stderr.decode()
         b = subprocess.run([harness] + oc.command_args(c, fa), capture_output=True)
         assert b.returncode == 0, b.stderr.decode()
-        assert oc.normalise(a.stdout, REF) == oc.normalise(b.stdout, harness), (seed, c["k"], c["m"], c["args"])
+        assert oc.ref_run_digest(b.stdout, harness, tmp_path) == want[c["name"]], (c["name"], c["k"], c["m"], c["args"])
 
 
 def test_errors(harness, tmp_path):
@@ -73,44 +70,26 @@ def test_errors(harness, tmp_path):
     assert r.returncode != 0 and "missing -k,--kmer option" in r.stderr
 
 
-DBG_REF = os.path.join(ROOT, "oracle", "_ref", "abyss-bloom-dbg-ref")
-
-
-@pytest.mark.skipif(not (os.path.exists(REF) and os.path.exists(DBG_REF)), reason="oracle/_ref not built")
-@pytest.mark.parametrize("k,m,fmt", [(32, 0, "--adj"), (32, 20, "--dot"), (48, 30, "--gfa1"), (64, 50, "--gfa2"), (96, 50, "--sam"), (40, 25, "--asqg")])
+@pytest.mark.parametrize("k,m,fmt", oc.UNITIG_RUNS)
 def test_real_unitig_sets(harness, tmp_path, k, m, fmt):
     # the pipeline of bin/abyss-pe on config 1 (SURVEY.md 8d: 53 333 x 150 bp reads of a 200 kbp genome): the reference's own
-    # unitig FASTA (tips, branches, blunt ends from coverage gaps) into both AdjList implementations
-    from abyss_b200.synth import ReadSet
-    rs = ReadSet(1, 200000, 53333, 150, 0.005)
-    fq = str(tmp_path / "r.fq")
-    rs.write_fastq(fq)
+    # unitig FASTA (tips, branches, blunt ends from coverage gaps) into AdjList, against the reference AdjList's output
+    text, sha = oc.unitig_set_fasta(k)
+    assert hashlib.sha256(text.encode()).hexdigest() == sha
+    assert text.count(">") > 10
     fa = str(tmp_path / "unitigs-1.fa")
-    subprocess.run(["bash", "-c", f"ulimit -s 65536; {DBG_REF} -k{k} --kc=2 -b64M -H4 -j1 {fq} > {fa} 2>/dev/null"], check=True)
-    n = sum(1 for line in open(fa) if line.startswith(">"))
-    assert n > 10
-    args = [f"-k{k}", f"-m{m}", fmt, fa]
-    a = subprocess.run([REF] + args, capture_output=True)
-    assert a.returncode == 0, a.stderr.decode()
-    b = subprocess.run([harness] + args, capture_output=True)
+    open(fa, "w").write(text)
+    b = subprocess.run([harness, f"-k{k}", f"-m{m}", fmt, fa], capture_output=True)
     assert b.returncode == 0, b.stderr.decode()
-    assert oc.normalise(a.stdout, REF) == oc.normalise(b.stdout, harness)
-    assert len(a.stdout) > 0
+    want = json.load(open(os.path.join(GOLD, "overlap_ref_runs.json")))[f"unitigs_config1_k{k}_m{m}_{fmt[2:]}"]
+    assert oc.ref_run_digest(b.stdout, harness, tmp_path) == want
+    assert want["bytes"] > 0
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref/AdjList-ref not built")
 def test_option_aliases_and_stdin(harness, tmp_path):
     # --gv = --dot, --gfa = --gfa1, -m0 = k-1, long options, several input files, contigs on standard input
-    c = oc.tiled_case(21, 20000, 31, 20)
-    half = len(c["records"]) // 2
-    a_fa, b_fa = str(tmp_path / "a.fa"), str(tmp_path / "b.fa")
-    oc.write_fasta(dict(c, records=c["records"][:half]), a_fa)
-    oc.write_fasta(dict(c, records=c["records"][half:]), b_fa)
-    both = open(a_fa).read() + open(b_fa).read()
-    for args, stdin in ((["--kmer=31", "--min-overlap=20", "--gv", a_fa, b_fa], None), (["-k31", "-m0", "--gfa", a_fa, b_fa], None),
-                        (["-k", "31", "-m", "25", "--SS", "--adj"], both), (["-k31", "--no-SS", "--asqg", "-"], both)):
-        ref = subprocess.run([REF] + args, input=stdin, capture_output=True, text=True)
-        assert ref.returncode == 0, ref.stderr
+    want = json.load(open(os.path.join(GOLD, "overlap_ref_runs.json")))
+    for name, args, stdin in oc.alias_runs(str(tmp_path)):
         got = subprocess.run([harness] + args, input=stdin, capture_output=True, text=True)
         assert got.returncode == 0, got.stderr
-        assert got.stdout == ref.stdout, args
+        assert oc.ref_run_digest(got.stdout.encode(), harness, tmp_path) == want[name], args

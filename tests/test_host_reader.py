@@ -4,6 +4,8 @@ while the GPU works on the previous batch -- must deliver exactly the records of
 boundaries fall: quality lines that start with '@', '+' or '>', multi-line FASTA, Casava headers, CRLF, a last line
 without newline, comment-led files (parsed serially), several files, compressed input."""
 import gzip
+import hashlib
+import json
 import os
 import random
 import subprocess
@@ -89,27 +91,36 @@ def test_stream_quality_options(exe, tmp_path):
         assert got == want
 
 
-REF_ARITH = os.path.join(ROOT, "oracle", "_ref", "ref_arith")
-
-
-@pytest.mark.skipif(not os.path.exists(REF_ARITH), reason="oracle/_ref not built (needs /root/reference)")
-def test_reader_equals_reference_reader(exe, tmp_path):
-    # the UNMODIFIED reference reader (DataLayer/FastaReader.cpp through oracle/_ref/ref_arith reads dump):
-    # ids (Casava suffix), chastity filter, masked-end trimming, case folding, multi-line FASTA, CRLF, gz
-    files = {"a.fq": fastq(2000, 11), "b.fq": fastq(1000, 12, crlf=True, casava=True), "c.fa": fasta(500, 13)}
+def write_files(d, files, gz_text=None):
     paths = []
     for name, text in files.items():
-        p = tmp_path / name
-        p.write_text(text, newline="")
-        paths.append(str(p))
-    gz = tmp_path / "g.fq.gz"
-    with gzip.open(gz, "wt", newline="") as f:
-        f.write(fastq(300, 14))
-    paths.append(str(gz))
-    ref = subprocess.run([REF_ARITH, "reads", "dump", *paths], capture_output=True, text=True)
-    assert ref.returncode == 0, ref.stderr
-    got, _ = run(exe, "stream", 3, 500, 4096, *paths)
-    assert got == ref.stdout
+        p = os.path.join(d, name)
+        with open(p, "w", newline="") as f:
+            f.write(text)
+        paths.append(p)
+    if gz_text is not None:
+        p = os.path.join(d, "g.fq.gz")
+        with gzip.open(p, "wt", newline="") as f:
+            f.write(gz_text)
+        paths.append(p)
+    return paths
+
+
+def reference_reader_inputs(d):
+    """ids (Casava suffix), chastity filter, masked-end trimming, case folding, multi-line FASTA, CRLF, gz"""
+    return write_files(d, {"a.fq": fastq(2000, 11), "b.fq": fastq(1000, 12, crlf=True, casava=True), "c.fa": fasta(500, 13)}, fastq(300, 14))
+
+
+def golden_digest(text):
+    return dict(sha256=hashlib.sha256(text.encode()).hexdigest(), lines=text.count("\n"))
+
+
+def test_reader_equals_reference_reader(exe, tmp_path, golden_dir):
+    # the output of the UNMODIFIED reference reader (DataLayer/FastaReader.cpp through oracle/_ref/ref_arith reads dump) on the
+    # same files (tests/golden/make_golden_reader.py)
+    want = json.load(open(os.path.join(golden_dir, "reader_cases.json")))["fastq_fasta_gz"]
+    got, _ = run(exe, "stream", 3, 500, 4096, *reference_reader_inputs(tmp_path))
+    assert golden_digest(got) == want
 
 
 def test_long_records(exe, tmp_path):
@@ -199,29 +210,33 @@ def qseq_text(n, seed, export=False):
     return "\n".join(out) + "\n"
 
 
-@pytest.mark.skipif(not os.path.exists(REF_ARITH), reason="oracle/_ref not built (needs /root/reference)")
-@pytest.mark.parametrize("opts", [{}, {"Q": "20"}, {"MASKQ": "15"}, {"NO_CHASTITY": "1"}, {"Q": "10", "QOFF": "64"}, {"MASKQ": "12", "QOFF": "33"},
-                                  {"NO_TRIM_MASKED": "1"}])
-def test_sam_qseq_export_equal_reference_reader(exe, tmp_path, opts):
+def format_inputs(d):
+    return write_files(d, {"a.sam": sam_text(800, 21), "b_qseq.txt": qseq_text(600, 22), "c_export.txt": qseq_text(400, 23, export=True),
+                           "d.fq": fastq(500, 24, casava=True), "e.fa": fasta(200, 25)})
+
+
+READER_OPTS = [{}, {"Q": "20"}, {"MASKQ": "15"}, {"NO_CHASTITY": "1"}, {"Q": "10", "QOFF": "64"}, {"MASKQ": "12", "QOFF": "33"}, {"NO_TRIM_MASKED": "1"}]
+
+
+def opts_key(opts):
+    return ",".join(f"{k}={v}" for k, v in opts.items()) or "default"
+
+
+@pytest.mark.parametrize("opts", READER_OPTS)
+def test_sam_qseq_export_equal_reference_reader(exe, tmp_path, golden_dir, opts):
     # the record formats of DataLayer/FastaReader.cpp:270-352 next to FASTQ, with the reader options of the command line
-    # (-q, -Q, --illumina-quality / --standard-quality, --no-chastity, --no-trim-masked), against the UNMODIFIED reference reader
-    files = {"a.sam": sam_text(800, 21), "b_qseq.txt": qseq_text(600, 22), "c_export.txt": qseq_text(400, 23, export=True),
-             "d.fq": fastq(500, 24, casava=True), "e.fa": fasta(200, 25)}
-    paths = []
-    for name, text in files.items():
-        p = tmp_path / name
-        p.write_text(text, newline="")
-        paths.append(str(p))
-    ref = subprocess.run([REF_ARITH, "reads", "dump", *paths], capture_output=True, text=True, env=dict(os.environ, **{"REF_" + k: v for k, v in opts.items()}))
-    assert ref.returncode == 0, ref.stderr
+    # (-q, -Q, --illumina-quality / --standard-quality, --no-chastity, --no-trim-masked), against the output of the UNMODIFIED
+    # reference reader on the same files with the same options (tests/golden/make_golden_reader.py)
+    want = json.load(open(os.path.join(golden_dir, "reader_cases.json")))["formats"][opts_key(opts)]
+    paths = format_inputs(tmp_path)
     env = {"READER_" + k: v for k, v in opts.items()}
     serial, _ = run(exe, "serial", *paths, env=env)
-    assert serial == ref.stdout
+    assert golden_digest(serial) == want
     got, _ = run(exe, "stream", 3, 250, 4096, *paths, env=env)
-    assert got == ref.stdout
+    assert got == serial
     got, _ = run(exe, "stream", 3, 250, 4096, *paths, env=dict(env, ABB_NO_MMAP="1"))
-    assert got == ref.stdout
-    assert ref.stdout.count("\n") > 1500
+    assert got == serial
+    assert want["lines"] > 1500
 
 
 @pytest.mark.parametrize("mapped", [True, False])
