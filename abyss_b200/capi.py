@@ -64,6 +64,10 @@ class SuccInfo(C.Structure):
     _fields_ = [("hash", C.c_uint64 * 4), ("mask", C.c_uint8), ("pad", C.c_uint8 * 7)]
 
 
+class Neighbourhood(C.Structure):
+    _fields_ = [("hash", C.c_uint64 * 9), ("attr", C.c_uint32 * 9), ("mask", C.c_uint16), ("pad", C.c_uint8 * 2)]
+
+
 class OverlapEdge(C.Structure):
     _fields_ = [("u", C.c_uint32), ("v", C.c_uint32), ("distance", C.c_int32)]
 
@@ -136,6 +140,7 @@ SIGNATURES = {
     "abb_filter_stream": (_vp, [_vp]),
     "abb_contains_reads": (C.c_int, [_vp, _vp, _vp, C.c_uint64, _vp, _vp, C.c_uint64, _u64p]),
     "abb_successors": (C.c_int, [_vp, _vp, C.c_uint64, C.c_uint, _vp, _vp, _vp]),
+    "abb_neighbours": (C.c_int, [_vp, _vp, C.c_uint, _vp, C.c_uint64, _vp]),
     "abb_overlap_create": (C.c_int, [C.POINTER(_vp), C.c_int]),
     "abb_overlap_destroy": (C.c_int, [_vp]),
     "abb_overlap_build": (C.c_int, [_vp, _vp, _vp, C.c_uint64, C.c_uint, C.c_uint, C.c_int, C.POINTER(C.POINTER(OverlapEdge)), _u64p]),
@@ -574,3 +579,16 @@ def successors(filt: "Filter", kmers, max_chain: int = 1):
     for i in range(n):
         out.append(([(info[i * max_chain + s].mask, list(info[i * max_chain + s].hash)) for s in range(ln[i])], self_h[i]))
     return out
+
+
+def neighbours(graph: "Filter", kmers, attrs=()):
+    """the k-mer and its 8 neighbours (abb_neighbours; vertex 0 = the k-mer, 1 + b = successor with last base b, 5 + b =
+    predecessor with first base b, b = A, C, G, T): for every k-mer (hashes[9], mask, attr[9]) -- canonical hashes, graph
+    membership (bit v = vertex v) and attribute bits (attr[v] bit j = attrs[j] contains vertex v)."""
+    lib = load()
+    ks = [s.encode() if isinstance(s, str) else bytes(s) for s in kmers]
+    n = len(ks)
+    out = (Neighbourhood * n)()
+    hs = (_vp * max(1, len(attrs)))(*[a.handle for a in attrs])
+    check(lib.abb_neighbours(graph.handle, hs, len(attrs), b"".join(ks), n, out))
+    return [(list(out[i].hash), out[i].mask, list(out[i].attr)) for i in range(n)]

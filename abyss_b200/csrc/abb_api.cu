@@ -903,6 +903,7 @@ int abb_filter_destroy(abb_filter* f)
 	f->gq_info.release();
 	f->gq_len.release();
 	f->gq_self.release();
+	f->gq_nb.release();
 	f->valid.release();
 	f->scan_tmp.release();
 	f->out8.release();
@@ -1395,6 +1396,56 @@ int abb_successors(abb_filter* f, const char* kmers, uint64_t n, unsigned max_ch
 		ABB_CUDA(cudaMemcpyAsync(out, d_info.p, n * max_chain * sizeof(abb_succ_info), cudaMemcpyDeviceToHost, f->stream));
 		ABB_CUDA(cudaMemcpyAsync(out_len, d_len.p, n * sizeof(unsigned), cudaMemcpyDeviceToHost, f->stream));
 		ABB_CUDA(cudaMemcpyAsync(self_hash, d_self.p, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, f->stream));
+		ABB_CUDA(cudaStreamSynchronize(f->stream));
+		return ABB_OK;
+	};
+	const int rc = run();
+	cudaStreamSynchronize(f->stream);
+	return rc;
+}
+
+int abb_neighbours(abb_filter* graph, abb_filter* const* attrs, unsigned n_attrs, const char* kmers, uint64_t n, abb_neighbourhood* out)
+{
+	abb_filter* const f = graph;
+	ABB_REQUIRE(f, "NULL filter");
+	ABB_REQUIRE(n_attrs <= 32, "at most 32 attribute filters, %u given", n_attrs);
+	ABB_REQUIRE(n_attrs == 0 || attrs, "NULL attribute filter list");
+	ABB_REQUIRE(f->mask.empty(), "graph neighbourhood queries are not available with a spaced seed");
+	ABB_REQUIRE(f->kind != ABB_COUNTING, "the graph of `abyss-bloom graph' is a bit or cascading filter, not a counting filter");
+	NbFilters F = {};
+	auto add = [&](const abb_filter* a, unsigned j) {
+		F.bits[j] = a->d_data + (uint64_t)(a->levels - 1) * a->bytes_per_level; // the last level: what the reference serialises
+		F.mod[j] = a->cfg.mod;
+		F.H[j] = a->H;
+		F.start[j + 1] = F.start[j] + 9 * a->H;
+	};
+	add(f, 0);
+	for (unsigned j = 0; j < n_attrs; ++j) {
+		const abb_filter* a = attrs[j];
+		ABB_REQUIRE(a, "NULL attribute filter %u", j);
+		ABB_REQUIRE(a->kind != ABB_COUNTING, "attribute filter %u is a counting filter", j);
+		ABB_REQUIRE(a->device == f->device, "attribute filter %u is on device %d, the graph on %d", j, a->device, f->device);
+		ABB_REQUIRE(a->H <= f->H, "attribute filter %u has %u hash functions, more than the graph's %u (it is probed with the graph's hash values)",
+		            j, a->H, f->H);
+		add(a, 1 + j);
+	}
+	F.n = 1 + n_attrs;
+	for (unsigned i = 0; i < kMaxHashes; ++i)
+		F.mult[i] = f->cfg.mult[i];
+	if (n == 0)
+		return ABB_OK;
+	ABB_REQUIRE(kmers && out, "NULL buffer");
+	ABB_CUDA(cudaSetDevice(f->device));
+	DevBuf<uint8_t>& d_k = f->gq_kmers;
+	DevBuf<abb_neighbourhood>& d_nb = f->gq_nb;
+	auto run = [&]() -> int {
+		ABB_CHECK(d_k.reserve(n * f->k));
+		ABB_CHECK(d_nb.reserve(n));
+		ABB_CUDA(cudaMemcpyAsync(d_k.p, kmers, n * f->k, cudaMemcpyHostToDevice, f->stream));
+		k_neighbours<<<blocks_for(n, kNbWarps), 32 * kNbWarps, 0, f->stream>>>(d_k.p, n, f->k, F, d_nb.p);
+		f->st.launches += 1;
+		ABB_CUDA(cudaGetLastError());
+		ABB_CUDA(cudaMemcpyAsync(out, d_nb.p, n * sizeof(abb_neighbourhood), cudaMemcpyDeviceToHost, f->stream));
 		ABB_CUDA(cudaStreamSynchronize(f->stream));
 		return ABB_OK;
 	};

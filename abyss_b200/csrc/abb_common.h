@@ -129,6 +129,7 @@ struct abb_filter {
 	abb::DevBuf<abb_succ_info> gq_info;
 	abb::DevBuf<unsigned> gq_len;
 	abb::DevBuf<uint64_t> gq_self;
+	abb::DevBuf<abb_neighbourhood> gq_nb; // abb_neighbours results (the k-mers go through gq_kmers)
 
 	// statistics
 	abb_insert_stats st = {};

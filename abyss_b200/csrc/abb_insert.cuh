@@ -1021,6 +1021,92 @@ k_successors(const uint8_t* __restrict__ kmers, uint64_t n, unsigned k, unsigned
 	len[w] = successors_chain(kmers + w * k, k, max_chain, probe, info + w * max_chain, self + w);
 }
 
+/** The bit filters k_neighbours probes: [0] the graph, [1..n) the attribute filters (last level of each).  Every filter is
+ *  probed with the graph's hash values -- its multipliers (mult, from the graph's k) and its first H[j] hashes -- modulo its
+ *  own size, as RollingBloomDBGVisitor::discover_vertex hands the graph vertex's getHashes() to each attribute filter. */
+constexpr unsigned kNbMaxFilters = 33;
+constexpr unsigned kNbWarps = 4;
+struct NbFilters {
+	const uint8_t* bits[kNbMaxFilters];
+	FastMod mod[kNbMaxFilters];
+	unsigned H[kNbMaxFilters];
+	unsigned start[kNbMaxFilters + 1]; // first probe of filter j in the flat probe list: 9 * (H[0] + .. + H[j-1])
+	unsigned n;
+	uint64_t mult[kMaxHashes];
+};
+
+/** the probe functor of neighbourhood() inside k_neighbours: the warp splits the 9 x sum(H) probes of one k-mer over its
+ *  lanes (lane = probe mod 32, as K4 lays 8 neighbours x 4 hash slots over a warp), issues four per lane before it looks at
+ *  any, and ORs the misses into one word per filter in shared memory (bit v = vertex v) */
+struct WarpNbProbe {
+	const NbFilters* F;
+	unsigned* fail; // [kNbMaxFilters] of this warp's shared memory, zero on entry
+	unsigned lane;
+	__device__ void operator()(const uint64_t* hash, unsigned* mask, uint32_t* attr) const
+	{
+		const unsigned total = F->start[F->n];
+		for (unsigned base = 0; base < total; base += 4 * 32) {
+			unsigned bit[4], slot[4];
+#pragma unroll
+			for (unsigned u = 0; u < 4; ++u) {
+				const unsigned p = base + 32 * u + lane;
+				slot[u] = ~0u;
+				bit[u] = 1;
+				if (p < total) {
+					unsigned j = 0;
+					while (F->start[j + 1] <= p)
+						++j;
+					const unsigned r = p - F->start[j], v = r / F->H[j], i = r - v * F->H[j];
+					uint64_t h0 = hash[0];
+#pragma unroll
+					for (unsigned w = 1; w < 9; ++w)
+						h0 = v == w ? hash[w] : h0;
+					const uint64_t t = h0 * F->mult[i]; // nth_hash with the graph's multipliers
+					const uint64_t x = i == 0 ? h0 : t ^ (t >> kMultiShift);
+					const uint64_t pos = fastmod_u64(x, F->mod[j]);
+					bit[u] = (__ldcg(F->bits[j] + (pos >> 3)) >> (pos & 7)) & 1;
+					slot[u] = j * 16 + v;
+				}
+			}
+#pragma unroll
+			for (unsigned u = 0; u < 4; ++u)
+				if (!bit[u])
+					atomicOr(&fail[slot[u] >> 4], 1u << (slot[u] & 15));
+		}
+		__syncwarp();
+		*mask = ~fail[0] & 0x1FFu;
+		const unsigned nA = F->n - 1;
+		const unsigned ok = lane < nA ? ~fail[1 + lane] : 0u; // lane j answers for attribute filter j
+#pragma unroll
+		for (unsigned v = 0; v < 9; ++v)
+			attr[v] = __ballot_sync(0xffffffffu, (ok >> v) & 1);
+	}
+};
+
+/** neighbourhoods of one breadth-first search level of `abyss-bloom graph`: one warp per k-mer; every lane computes the 9
+ *  hashes (neighbourhood(), abb_graph.cuh), the warp probes the graph and attribute filters for all 9 vertices at once --
+ *  one round trip to memory per k-mer instead of the reference's sequence of 8 x H dependent lookups */
+__global__ void __launch_bounds__(32 * kNbWarps)
+k_neighbours(const uint8_t* __restrict__ kmers, uint64_t n, unsigned k, const __grid_constant__ NbFilters F,
+             abb_neighbourhood* __restrict__ out)
+{
+	__shared__ unsigned s_fail[kNbWarps][kNbMaxFilters];
+	const unsigned warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+	const uint64_t w = (uint64_t)blockIdx.x * kNbWarps + warp;
+	if (w >= n)
+		return;
+	s_fail[warp][lane] = 0;
+	if (lane == 0)
+		s_fail[warp][32] = 0;
+	__syncwarp();
+	const WarpNbProbe probe = { &F, s_fail[warp], lane };
+	abb_neighbourhood r;
+	neighbourhood(kmers + w * k, k, probe, &r);
+	r.pad[0] = r.pad[1] = 0;
+	if (lane == 0)
+		out[w] = r;
+}
+
 /** popCount / filtered_popcount (CountingBloomFilter.hpp:219-244) and getPop (BloomFilter.hpp:313-320) */
 static __global__ void __launch_bounds__(256)
 k_popcount(const uint8_t* __restrict__ data, uint64_t nbytes, int counting, unsigned threshold,

@@ -277,6 +277,23 @@ typedef struct abb_succ_info {
 int abb_successors(abb_filter* f, const char* kmers, uint64_t n, unsigned max_chain, abb_succ_info* out, unsigned* out_len,
                    uint64_t* self_hash);
 
+/* ---- neighbourhoods of graph vertices, for `abyss-bloom graph` (Bloom/bloom.cc:983-1153; out_edge_iterator / in_edge_iterator,
+ * BloomDBG/RollingBloomDBG.h:300-453): for each of n k-mers (n * k characters, hashed as the reference hashes any character:
+ * either case, non-ACGT as ntHash's seedTab gives it) the k-mer and its 8 neighbours.  Vertex v = 0: the k-mer itself;
+ * v = 1 + b: its successor (shifted left, last base b = A, C, G, T); v = 5 + b: its predecessor (shifted right, first base b).
+ * hash[v]: canonical ntHash (vertex identity).  mask bit v: the graph filter contains vertex v (all bits of its last level).
+ * attr[v] bit j: attribute filter attrs[j] contains vertex v, probed with the GRAPH's hash values (its k and its first
+ * H_j hashes) modulo the attribute filter's own size (RollingBloomDBGVisitor.h:122-131).  Bit and cascading filters only;
+ * n_attrs <= 32, each attribute filter on the graph's device with at most as many hashes as the graph; no spaced seed. */
+typedef struct abb_neighbourhood {
+	uint64_t hash[9];
+	uint32_t attr[9];
+	uint16_t mask;
+	uint8_t pad[2];
+} abb_neighbourhood;
+int abb_neighbours(abb_filter* graph, abb_filter* const* attrs, unsigned n_attrs, const char* kmers, uint64_t n,
+                   abb_neighbourhood* out);
+
 /* ---- the next stage: contig overlap graph (AdjList/AdjList.cpp:140-291; bin/abyss-pe:577 runs it on the unitig FASTA) ----
  * Vertices are ContigNode indices (Common/ContigNode.h): 2*i = contig i as given, 2*i+1 = its reverse complement.
  * Edges u -> v: the last `overlap` bases of u equal the first `overlap` bases of v; distance = -overlap.
